@@ -288,6 +288,27 @@ def verify_against_oracle(cfg, start, n, path_bytes, path_off, json_bytes, json_
             "seconds": round(time.perf_counter() - t0, 2)}
 
 
+# ------------------------------------------------------------------------------------------- dumps
+
+DUMP_SEED = 20251017
+DUMP_CAP = {"bytes": (4 << 20, np.float32), "off": (1 << 20, np.float64)}    # elements, dtype: 48 MiB in all
+
+
+def dump_outputs(out_dir, dev, arrays):
+    """Write the outputs of the last timed step as out_dir/<name>.npy, so that two builds run with the same arguments
+    can be compared output for output.  `arrays`: name -> device tensor (uint8 byte stream or int64 offsets); byte
+    values go out as float32 and offsets as float64, both exactly.  An array longer than its cap is written as a
+    fixed, seeded sample of its elements in index order (the same indices for the same length)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        cap, dtype = DUMP_CAP["bytes" if t.dtype == torch.uint8 else "off"]
+        if t.numel() > cap:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(t.numel(), cap, replace=False))
+            t = t[torch.from_numpy(idx).to(dev)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(dtype))
+
+
 # ---------------------------------------------------------------------------------------- GPU arm
 
 class Rig:
@@ -336,6 +357,17 @@ def roof(rig, name, nbytes, ms, launches, time_every, traffic):
             "timing": "CUDA events around the launch on every %s step of the timed region" % (
                 "" if time_every == 1 else "%d-th" % time_every),
             "peak_source": rig.peak_src}
+
+
+def device_outputs(res, dev):
+    """The byte streams and offset arrays of a finished REGK_OUT_DEVICE result as device tensors, by name."""
+    import torch
+    from registrar_b200 import multigpu
+    n = int(res.n)
+    return {"path_bytes": multigpu.device_tensor(res.path_bytes, int(res.path_total), torch.uint8, dev),
+            "path_off": multigpu.device_tensor(res.path_off, n + 1, torch.int64, dev),
+            "json_bytes": multigpu.device_tensor(res.json_bytes, int(res.json_total), torch.uint8, dev),
+            "json_off": multigpu.device_tensor(res.json_off, n + 1, torch.int64, dev)}
 
 
 def device_resident(rig, host_batches):
@@ -415,9 +447,10 @@ def e2e_loop(rig, pinned, steps, depth=2):
     return dt, h2d, d2h
 
 
-def measure_single(rig, cfg, n, start, steps, warmup, e2e_steps, time_every, verify=True):
-    """One configuration on this rank's GPU alone: value arm, e2e arm, per-kernel roofline, output check."""
-    from registrar_b200 import multigpu, synth
+def measure_single(rig, cfg, n, start, steps, warmup, e2e_steps, time_every, verify=True, dump=None):
+    """One configuration on this rank's GPU alone: value arm, e2e arm, per-kernel roofline, output check.
+    dump: directory for the outputs of the last timed step (dump_outputs)."""
+    from registrar_b200 import synth
     torch, ctx = rig.torch, rig.ctx
     NB = 4 if n <= 2_000_000 else 2
     host_batches = [synth.generate(cfg, n=n, start=start + b * n) for b in range(NB)]
@@ -431,16 +464,14 @@ def measure_single(rig, cfg, n, start, steps, warmup, e2e_steps, time_every, ver
     ctx.set_option("time_every", 1)
     last = stats["last"]
     path_total, json_total = int(last.path_total), int(last.json_total)
+    if dump:
+        dump_outputs(dump, rig.dev, device_outputs(last, rig.dev))      # before the next call overwrites them
 
     verified = None
     if verify:
         # one more, synchronous run of batch 0: its device result against the oracle
-        r = ctx.register_raw(cbatches[0])
-        pb = multigpu.device_tensor(r.path_bytes, int(r.path_total), torch.uint8, rig.dev)
-        jb = multigpu.device_tensor(r.json_bytes, int(r.json_total), torch.uint8, rig.dev)
-        po = multigpu.device_tensor(r.path_off, n + 1, torch.int64, rig.dev)
-        jo = multigpu.device_tensor(r.json_off, n + 1, torch.int64, rig.dev)
-        verified = verify_against_oracle(cfg, start, n, pb, po, jb, jo)
+        o = device_outputs(ctx.register_raw(cbatches[0]), rig.dev)
+        verified = verify_against_oracle(cfg, start, n, o["path_bytes"], o["path_off"], o["json_bytes"], o["json_off"])
 
     # ---- end-to-end arm: host buffers through the public call ----
     del cbatches, keep
@@ -483,8 +514,9 @@ def json_capacity(hb, max_type_len=13):
     return hb.n * (38 + 2 * max_type_len + 4 + 18 + 11) + 2 * int(hb.addr_off[-1]) + 11 * int(hb.ports_off[-1]) + 16
 
 
-def measure_job(rig, cfg, n_total, steps, warmup, e2e_steps, verify=True):
-    """N > 1: the job sharded over the ranks, reassembled on every rank inside the timed region (fused push)."""
+def measure_job(rig, cfg, n_total, steps, warmup, e2e_steps, verify=True, dump=None):
+    """N > 1: the job sharded over the ranks, reassembled on every rank inside the timed region (fused push).
+    dump: directory for rank 0's copy of the whole job's outputs of the last timed step (dump_outputs)."""
     from registrar_b200 import multigpu, synth
     torch, ctx, dist = rig.torch, rig.ctx, rig.dist
     lo, hi = multigpu.shard_range(n_total, rig.rank, rig.world)
@@ -509,6 +541,10 @@ def measure_job(rig, cfg, n_total, steps, warmup, e2e_steps, verify=True):
     ctx.set_option("async", 0)
     last = st_job["last"]
     recv = job.nbytes_received(last)
+    if dump and rig.rank == 0:
+        g = job.result(last)
+        dump_outputs(dump, rig.dev, {"path_bytes": g.path_bytes, "path_off": g.path_off, "json_bytes": g.json_bytes,
+                                     "json_off": g.json_off})
     verified = None
     if verify:
         # every rank checks ITS OWN copy of the gathered streams on its own record range against the CPU oracle (the
@@ -602,7 +638,7 @@ def run_b200(args):
     e2e_steps = 0 if args.e2e_steps <= 0 and rig.world > 1 else max(3, min(args.steps, args.e2e_steps))
     if rig.world == 1:
         m = measure_single(rig, cfg, n, 0, args.steps, args.warmup, e2e_steps, time_every=1 if n > 2_000_000 else 8,
-                           verify=not args.no_verify)
+                           verify=not args.no_verify, dump=args.dump_outputs)
         extras = {}
         if not args.only_headline:
             for xcfg, xn in EXTRAS:
@@ -616,7 +652,8 @@ def run_b200(args):
                 extras["%s_%d" % (xcfg, xn)] = x
         scaling = "strong"
     else:
-        m = measure_job(rig, cfg, n, args.steps, args.warmup, e2e_steps, verify=not args.no_verify)
+        m = measure_job(rig, cfg, n, args.steps, args.warmup, e2e_steps, verify=not args.no_verify,
+                        dump=args.dump_outputs)
         extras = {}
         scaling = "strong"
     rig.sampler.stop_flag = True
@@ -705,19 +742,13 @@ def run_reference(args):
     from registrar_b200 import synth
     n, cfg = args.records, args.config
     batch = synth.generate(cfg, n=n, start=0)
-    steps = max(args.steps, 1)
     from oracle import oracle
     threads, rates = oracle.calibrate_threads(batch)        # same choice of thread count as the b200 arm's cpu_baseline
     for _ in range(max(min(args.warmup, 3), 1)):
         oracle.register_batch(batch, threads=threads, timing_only=True)
-    budget = time.perf_counter() + 120.0
-    done, total_s = 0, 0.0
-    for _ in range(min(steps, 200)):
-        r = oracle.register_batch(batch, threads=threads, timing_only=True)
-        total_s += r.seconds
-        done += 1
-        if time.perf_counter() > budget:
-            break
+    done, total_s = args.steps, 0.0
+    for _ in range(done):
+        total_s += oracle.register_batch(batch, threads=threads, timing_only=True).seconds
     value = n * done / total_s
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": done, "warmup": args.warmup,
@@ -751,7 +782,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-verify", action="store_true", help="skip the oracle fingerprint check (profiling runs)")
     ap.add_argument("--only-headline", action="store_true", help="N=1: skip the extra configurations")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (large ones as a seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

@@ -1,10 +1,10 @@
 """Generate the committed golden fixtures by EXECUTING the reference.
 
-Runs only in the build container (needs /root/reference to have built oracle/_ref/regref via
-`make -C oracle ref`): the unmodified /root/reference/lib/register.js is evaluated on the
-SpiderMonkey engine of the reference tree with a recording fake ZooKeeper client, and what it passes
-to zk.create()/zk.put() is stored next to the inputs.
+Needs oracle/_ref/regref, built from a checkout of the reference: the unmodified lib/register.js of that
+checkout is evaluated on the SpiderMonkey engine of its tree with a recording fake ZooKeeper client, and
+what it passes to zk.create()/zk.put() is stored next to the inputs.
 
+    make -C oracle ref REF=<reference checkout>
     python tests/golden/make_golden.py
 
 Outputs (tests/golden/):
@@ -14,6 +14,10 @@ Outputs (tests/golden/):
                   shapes, the reference's README / test-suite inputs); same schema
   calls.jsonl     full call traces of register() for alias / service registrations:
                   {"in": record, "calls": [[op, ...], ...]}
+  reference_runs.jsonl
+                  the host nodes of synthetic batches (REFERENCE_RUNS) as 64-bit digests, one line per batch:
+                  {"config", "start", "n", "inputs": digest of the harness input text,
+                   "path": [digest per record], "json": [digest per record]}
 """
 import json
 import os
@@ -22,9 +26,15 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(HERE))
 
+from golden_util import digest, inputs_digest  # noqa: E402
 from oracle import refrun  # noqa: E402
 from registrar_b200 import synth  # noqa: E402
+
+# (config, start, n) of the synthetic batches tests/test_reference_live.py compares with the reference
+REFERENCE_RUNS = [("config1", 5000, 400), ("config3", 123456, 400), ("config5", 77, 400),
+                  ("config1", 9000, 600), ("config3", 654321, 600), ("config5", 4242, 600)]
 
 
 def rec_json(r):
@@ -83,7 +93,7 @@ def call_records():
 
 def main():
     if not refrun.available():
-        raise SystemExit("oracle/_ref/regref is missing: run `make -C oracle ref` (needs /root/reference)")
+        raise SystemExit("oracle/_ref/regref is missing: run `make -C oracle ref REF=<reference checkout>`")
     # config1: records as the product sees them (bytes fields decoded as latin-1 == ASCII here)
     b = synth.generate("config1")
     recs = [b.record(i) for i in range(b.n)]
@@ -103,6 +113,14 @@ def main():
     with open(os.path.join(HERE, "calls.jsonl"), "w") as f:
         for r, calls in zip(recs, traces):
             f.write(json.dumps({"in": rec_json(r), "calls": calls}, separators=(",", ":")) + "\n")
+    with open(os.path.join(HERE, "reference_runs.jsonl"), "w") as f:
+        for config, start, n in REFERENCE_RUNS:
+            b = synth.generate(config, n=n, start=start)
+            recs = [b.record(i) for i in range(b.n)]
+            outs = refrun.host_records(recs)
+            f.write(json.dumps({"config": config, "start": start, "n": n, "inputs": inputs_digest(recs),
+                                "path": [digest(p) for p, _ in outs], "json": [digest(j) for _, j in outs]},
+                               separators=(",", ":")) + "\n")
     print("golden fixtures written:", [x for x in sorted(os.listdir(HERE)) if x.endswith(".jsonl")])
 
 

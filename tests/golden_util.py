@@ -1,10 +1,22 @@
 """Load the committed golden fixtures (tests/golden/*.jsonl; produced by tests/golden/make_golden.py from the
 reference's own lib/register.js)."""
+import hashlib
 import json
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 HARNESS_INTERFACE_ADDRESS = "10.77.77.7"
+
+
+def digest(b: bytes) -> str:
+    """64-bit digest of one output (reference_runs.jsonl stores these instead of the bytes)."""
+    return hashlib.blake2b(b, digest_size=8).hexdigest()
+
+
+def inputs_digest(records) -> str:
+    """Digest of the harness input text of `records`: pins the inputs a stored reference run was made from."""
+    from oracle import refrun
+    return digest("\n".join(refrun.opts_line(r) for r in records).encode("ascii"))
 
 
 def load(name):

@@ -1,5 +1,5 @@
 import os, sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from registrar_b200 import _native, synth
 ctx = _native.Context(0); ctx.set_option("chunk_records", 0)
 b = synth.generate("config3", n=2_000_000)
